@@ -26,6 +26,16 @@ state spends 30-100) on a = b = 1024, d = 2, w = 5: 24 x 86.7 GFLOP.
 grows ("scaling": "strong").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+                  [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy
+(N = 1: the 1x1 norm environment <psi|psi>; N > 1: the Ritz value and the
+gathered Ritz vector), so that two builds can be compared output for output:
+the inputs are generated from fixed seeds.  For N = 1 that is one number,
+because a caller of the MPS-norm path receives nothing else; it still depends
+on every one of the 400 contractions of the step.  The CPU arm
+(`--impl reference`) times a sample of the workload and has no outputs to
+dump, so the two options are rejected together.
 
 `--impl reference` times the reference's own CPU path for the same config
 (the numpy/OpenBLAS restatement in oracle/ -- the reference is pure Python +
@@ -335,7 +345,7 @@ def run_unit(qb, shard, prob, steps, warmup, barrier, events=True):
     assert nmv == UNIT_MATVECS, nmv
     if shard is not None:
         shard.check()           # a peer-memory kernel that gave up waiting would show here
-    return ev0.elapsed_time(ev1) / steps, theta, H
+    return ev0.elapsed_time(ev1) / steps, theta, x, H
 
 
 def time_exchange(shard, prob, reps=20):
@@ -357,6 +367,15 @@ def time_exchange(shard, prob, reps=20):
     return e0.elapsed_time(e1) / reps
 
 
+def dump_outputs(dirname, arrays):
+    """Write each array as DIR/<name>.npy (float32 / float64 only)."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -368,7 +387,13 @@ def main():
     ap.add_argument("--no-dmrg", action="store_true")
     ap.add_argument("--exchange", default=os.environ.get("QB_EXCHANGE", "auto"),
                     help="N>1: auto | p2p | nccl")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path, not --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -429,8 +454,14 @@ def bench_sharded(args, qb, _lib, dist, dev, rank, local_rank, world, barrier, m
     if rank == 0:
         sampler.start()
     n0 = _lib.launch_count()
-    ms, theta, H = run_unit(qb, shard, prob, args.steps, args.warmup, barrier)
+    ms, theta, x, H = run_unit(qb, shard, prob, args.steps, args.warmup, barrier)
     launches = _lib.launch_count() - n0
+    if args.dump_outputs:
+        x_full = H.gather(x).to_numpy()          # collective: every rank takes part
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"eigensolve_theta": np.array([theta]),
+                                             "eigensolve_x": x_full})
+        del x_full
     clocks = sampler.stop() if rank == 0 else None
     ms_max = max_over_ranks(ms)
     value = flops / (ms_max * 1e-3) / 1e12
@@ -441,7 +472,7 @@ def bench_sharded(args, qb, _lib, dist, dev, rank, local_rank, world, barrier, m
     # N=1 point of the strong-scaling curve, measured next to the N-rank run
     single_ms = None
     if rank == 0:
-        single_ms, theta1, _ = run_unit(qb, None, prob, max(2, args.steps // 2), 2,
+        single_ms, theta1, _, _ = run_unit(qb, None, prob, max(2, args.steps // 2), 2,
                                         torch.cuda.synchronize)
         assert abs(theta1 - theta) <= 1e-9 * abs(theta), (theta1, theta)
     barrier()
@@ -571,6 +602,8 @@ def bench_mps_norm(args, qb, _lib, dev, barrier):
     ms_max = ev0.elapsed_time(ev1) / args.steps
     value = flops / (ms_max * 1e-3) / 1e12
     norm2 = float(out.reshape(()).item())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mps_norm2": out.to_numpy()})
 
     # dominant kernel: the full-size (chi x chi.d x chi) contraction launches
     big = [(a.elapsed_time(b), fl) for a, b, fl, l, r in records if l == CHI and r == CHI]
@@ -648,7 +681,7 @@ def bench_mps_norm(args, qb, _lib, dev, barrier):
 
     # ---- the unit the multi-GPU line shards, unsharded on this GPU -----------
     prob = build_unit_problem(qb, dev)
-    unit_ms, theta, H = run_unit(qb, None, prob, max(2, args.steps // 2), 2, barrier)
+    unit_ms, theta, _, H = run_unit(qb, None, prob, max(2, args.steps // 2), 2, barrier)
     unit_flops = UNIT_MATVECS * matvec_flops()
     shard_unit = {"workload": config_shard(1)["workload"], "ms_per_step": unit_ms,
                   "tflops": unit_flops / (unit_ms * 1e-3) / 1e12,

@@ -752,10 +752,226 @@ def mps_dmrg_cases():
     json.dump(meta, open(os.path.join(OUT, "mps_dmrg.json"), "w"), indent=1)
 
 
+DROPIN_SPLITS = [
+    ("svd", dict(cutoff=1e-3, cutoff_mode="rel")), ("svd", dict(max_bond=3, absorb="left")),
+    ("svd:eig", dict(max_bond=4)), ("qr", {}), ("lq", {}), ("eigh", dict(max_bond=4)),
+    ("polar_right", {}), ("polar_left", {}),
+]
+
+
+def dropin_cases():
+    """What the drop-in tests compare the backend with: the names the
+    reference's composed drivers accept registrations for, and its own numpy
+    runs of Tensor @ / tensor_contract / Tensor.split and of the drivers
+    either side of the hot path, with the inputs they ran on."""
+    import warnings
+    from quimb.linalg import base_linalg
+    from quimb.tensor import array_ops
+    store, meta = {}, {}
+    meta["registrable"] = {
+        "decomp": sorted(nm for nm, f in vars(decomp).items() if hasattr(f, "register")),
+        "array_ops": sorted(nm for nm, f in vars(array_ops).items() if hasattr(f, "register")),
+        "split_values": sorted(decomp._SPLIT_VALUES_FNS),
+        "eigs_methods": sorted(base_linalg._EIGS_METHODS),
+    }
+    rng = np.random.default_rng(0)
+    shapes = {"a": ((4, 5, 6), "abc"), "b": ((6, 5, 7), "cbd"), "c": ((7, 3), "de"),
+              "h1": ((3, 4), "xh"), "h2": ((4, 5), "hy"), "h3": ((4, 2), "hz")}
+    ts = {}
+    for k, (shape, inds) in shapes.items():
+        store[f"contract__{k}"] = rng.standard_normal(shape)
+        ts[k] = qtn.Tensor(store[f"contract__{k}"], inds=inds)
+    for k, (shape, inds) in {"z1": ((3, 4), "ab"), "z2": ((4, 3), "ba")}.items():
+        store[f"contract__{k}"] = rng.standard_normal(shape) + 1j * rng.standard_normal(shape)
+        ts[k] = qtn.Tensor(store[f"contract__{k}"], inds=inds)
+    meta["contract_inds"] = {k: list(t.inds) for k, t in ts.items()}
+    ab = ts["a"] @ ts["b"]
+    store["contract__ab"] = np.asarray(ab.data)
+    meta["contract_ab_inds"] = list(ab.inds)
+    store["contract__abc_ea"] = np.asarray(
+        qtn.tensor_contract(ts["a"], ts["b"], ts["c"], output_inds="ea").data)
+    store["contract__hyper_xyz"] = np.asarray(
+        qtn.tensor_contract(ts["h1"], ts["h2"], ts["h3"], output_inds="xyz").data)
+    z = complex(qtn.tensor_contract(ts["z1"], ts["z2"]))
+    m, e = qtn.tensor_contract(ts["z1"], ts["z2"], strip_exponent=True)
+    meta["contract_z"] = [z.real, z.imag]
+    meta["contract_z_strip"] = {"mantissa": [complex(m).real, complex(m).imag],
+                                "exponent": float(e)}
+    splits = []
+    for k, (method, kw) in enumerate(DROPIN_SPLITS):
+        rng = np.random.default_rng(1)
+        x = rng.standard_normal((6, 4, 5))
+        if method == "eigh":
+            y = rng.standard_normal((6, 4, 6, 4))
+            x = y + y.transpose(2, 3, 0, 1)
+            inds, left = "abcd", ["a", "b"]
+        else:
+            inds = "abc"
+            left = ["a", "b"] if method in ("qr", "polar_right") else ["a"]
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            ref = qtn.Tensor(x, inds=inds).split(left_inds=left, method=method,
+                                                 get="arrays", **kw)
+        store[f"split{k}__x"] = x
+        store[f"split{k}__product"] = np.tensordot(ref[0], ref[-1], 1)
+        splits.append({"method": method, "kw": kw, "inds": inds, "left_inds": left,
+                       "shapes": [list(r.shape) for r in ref]})
+    meta["splits"] = splits
+    _dropin_callers(store, meta)
+    np.savez_compressed(os.path.join(OUT, "dropin.npz"), **store)
+    json.dump(meta, open(os.path.join(OUT, "dropin.json"), "w"), indent=1)
+
+
+def _store_tn(tn, key, store):
+    """Every tensor of a network: data under key__t<k>, index names returned."""
+    inds = []
+    for k, t in enumerate(tn.tensors):
+        store[f"{key}__t{k}"] = np.asarray(t.data)
+        inds.append(list(map(str, t.inds)))
+    return inds
+
+
+def _dropin_callers(store, meta):
+    """The reference's drivers either side of the hot path, on numpy: MPS
+    canonize / compress / expectation, TNLinearOperator, DMRG2 (both local
+    eigensolver forms), boundary contraction, circuit amplitude, TEBD, DMRG1,
+    MPS gates / MPO application / addition / entropy, compressed contraction."""
+    import warnings
+    from quimb.tensor.tensor_core import TNLinearOperator
+    warnings.simplefilter("ignore")
+
+    def sites(p, key):
+        for i in range(p.L):
+            store[f"{key}__{i}"] = np.asarray(p[i].data)       # 'lrp', ends (r,p)/(l,p)
+
+    def mpo(H, key):
+        for i in range(H.L):
+            store[f"{key}__{i}"] = np.asarray(H[i].data)       # 'lrud'
+
+    # canonize / compress / expectation / linear operator
+    p = qtn.MPS_rand_state(6, 7, seed=4)
+    sites(p, "canon_p")
+    c = {"norm0": float(p.H @ p)}
+    p.left_canonize()
+    c["norm_canon"] = float(p.H @ p)
+    p.compress(max_bond=3)
+    c["norm_compressed"] = float(p.H @ p)
+    c["max_bond"] = int(p.max_bond())
+    H = qtn.MPO_ham_heis(6)
+    mpo(H, "heis6")
+    c["expec"] = float(qtn.expec_TN_1D(p.H, H, p))
+    rng = np.random.default_rng(2)
+    ts = [qtn.Tensor(rng.standard_normal((5, 3, 5)), inds=("a", "w", "b"), tags="L"),
+          qtn.Tensor(rng.standard_normal((3, 2, 2)), inds=("w", "p", "q"), tags="W")]
+    A = TNLinearOperator(ts, left_inds=("a", "p"), right_inds=("b", "q"))
+    v = rng.standard_normal(10)
+    for k, t in enumerate(ts):
+        store[f"linop__t{k}"] = np.asarray(t.data)
+    store["linop__v"] = v
+    store["linop__matvec"] = A.matvec(v)
+    store["linop__dense"] = A.to_dense()
+    meta["canon"] = c
+
+    # DMRG2, L = 8: quimb's default eigensolver path and both dense settings
+    L = 8
+    H8 = qtn.MPO_ham_heis(L)
+    mpo(H8, "heis8")
+    p4 = qtn.MPS_rand_state(L, 4, seed=3)
+    p8 = qtn.MPS_rand_state(L, 8, seed=3)
+    sites(p4, "dmrg_p4")
+    sites(p8, "dmrg_p8")
+    d = {}
+    ref = qtn.DMRG2(H8.copy(), bond_dims=[8, 16, 32], cutoffs=1e-10, p0=p4.copy())
+    ref.solve(tol=1e-8, max_sweeps=5, verbosity=0)
+    d["default_energy"] = float(ref.energy)
+    for dense in (True, False):
+        ref = qtn.DMRG2(H8.copy(), bond_dims=[8, 16], cutoffs=1e-10, p0=p8.copy())
+        ref.opts["local_eig_ham_dense"] = dense
+        ref.solve(tol=1e-9, max_sweeps=5, verbosity=0)
+        d[f"dense_{dense}"] = {"energy": float(ref.energy),
+                               "bonds": [int(ref.state.bond_size(i, i + 1)) for i in range(L - 1)]}
+    d["exact"] = float(qu.groundenergy(qu.ham_heis(L, cyclic=False, sparse=True)))
+    r1 = qtn.DMRG1(H8.copy(), bond_dims=[8, 16], p0=p8.copy())
+    r1.solve(tol=1e-8, max_sweeps=4, verbosity=0)
+    d["dmrg1_energy"] = float(r1.energy)
+    meta["dmrg"] = d
+
+    cl = {}
+    # PEPS norm by boundary-MPS contraction; classical Ising partition function
+    peps = qtn.PEPS.rand(4, 4, bond_dim=2, seed=1, dtype="complex128")
+    for i in range(4):
+        for j in range(4):
+            store[f"peps__{i}_{j}"] = np.asarray(peps[i, j].data)
+    v = complex(peps.make_norm().contract_boundary(max_bond=8, cutoff=0.0,
+                                                   layer_tags=("KET", "BRA")))
+    cl["peps_norm"] = [v.real, v.imag]
+    ising = qtn.TN2D_classical_ising_partition_function(4, 4, beta=0.3)
+    cl["ising_tensors"] = _dump_tn2d(ising, "ising", store)
+    cl["ising_Z"] = float(ising.contract_boundary(max_bond=8))
+
+    # circuit amplitude
+    rng = np.random.default_rng(0)
+    circ = qtn.Circuit(5)
+    for dd in range(4):
+        for q in range(5):
+            circ.apply_gate("U3", *rng.uniform(0, 6, 3), q)
+        for q in range(dd % 2, 4, 2):
+            circ.apply_gate("CZ", q, q + 1)
+    amp = complex(circ.amplitude("01001"))
+    cl["amp_01001"] = [amp.real, amp.imag]
+    # the networks unsimplified: quimb's default simplification reduces these
+    # to the amplitude itself, which would leave nothing to contract
+    cl["amp_01001_inds"] = _store_tn(circ.amplitude_tn("01001", simplify_sequence=""),
+                                     "amp_01001", store)
+    tn = circ.amplitude_tn("00000", simplify_sequence="")
+    cl["amp_00000_inds"] = _store_tn(tn, "amp_00000", store)
+    amp = complex(tn.full_simplify() ^ all)
+    cl["amp_00000"] = [amp.real, amp.imag]
+
+    # TEBD from the Neel state
+    ham = qtn.ham_1d_heis(6)
+    store["tebd__h2"] = np.asarray(ham.terms[(0, 1)])
+    cl["tebd_terms_equal"] = all(np.allclose(ham.terms[k], ham.terms[(0, 1)]) for k in ham.terms)
+    t0 = qtn.TEBD(qtn.MPS_neel_state(6), ham, progbar=False)
+    t0.update_to(0.2, dt=0.05, order=2)
+    store["tebd__dense"] = np.asarray(t0.pt.to_dense()).reshape(-1)
+
+    # MPS gates, MPO application, addition, entropy
+    p = qtn.MPS_rand_state(6, 4, seed=2)
+    q = qtn.MPS_rand_state(6, 3, seed=6)
+    sites(p, "gates_p")
+    sites(q, "gates_q")
+    G = qu.rand_uni(4, seed=1).reshape(2, 2, 2, 2)
+    store["gates__G"] = np.asarray(G)
+    for where, fn in (((2, 3), "gate_split"), ((0, 4), "gate_with_auto_swap")):
+        store[f"gates__{fn}"] = np.asarray(getattr(p, fn)(G, where, cutoff=1e-12).to_dense()).reshape(-1)
+    store["gates__apply"] = np.asarray(H.apply(p).to_dense()).reshape(-1)
+    store["gates__add"] = np.asarray((p + q).to_dense()).reshape(-1)
+    cl["entropy3"] = float(p.entropy(3))
+    meta["callers"] = cl
+
+    # compressed contraction along an inward sequence; max_bond below D, so
+    # that every run truncates (the value differs from the exact contraction)
+    tn = qtn.TN2D_rand(4, 4, D=4, seed=5)
+    tids = list(tn.tensor_map)
+    for k, t in enumerate(tids):
+        store[f"compressed__t{k}"] = np.asarray(tn.tensor_map[t].data)
+    seq_pos = [(i, i + 1) for i in range(len(tids) - 1)]
+    seq = [(tids[a], tids[b]) for a, b in seq_pos]
+    runs = []
+    for kw in (dict(max_bond=3, cutoff=0.0, tree_gauge_distance=0, compress_mode="basic"),
+               dict(max_bond=3, cutoff=1e-8, tree_gauge_distance=0, compress_mode="basic",
+                    compress_late=False)):
+        val = tn.copy()._contract_compressed_tid_sequence(seq, output_inds=(), **kw)
+        runs.append({"kw": kw, "value": float(val)})
+    meta["compressed"] = {"inputs": [list(map(str, tn.tensor_map[t].inds)) for t in tids],
+                          "seq": seq_pos, "runs": runs, "exact": float(tn.contract(all))}
+
+
 if __name__ == "__main__":
     only = set(sys.argv[1:])
     for fn in (contract_cases, decomp_cases, decomp2_cases, decomp3_cases, boundary_cases, compressed_cases,
-               tebd_cases, mps_ops_cases, mps_dmrg_cases):
+               tebd_cases, mps_ops_cases, mps_dmrg_cases, dropin_cases):
         if not only or fn.__name__ in only:
             fn()
     print("golden fixtures written to", OUT)
